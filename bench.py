@@ -1,8 +1,8 @@
 #!/usr/bin/env python3
 """Headline benchmark: PyTorch-GPU recipe retarget, ResNet-50 training images/sec.
 
-Contract (driver): ``python bench.py --gpus N --steps K --warmup W`` (N>1 under
-torchrun, one rank per GPU).  Prints ONE JSON line on rank 0.
+Usage: ``python bench.py --gpus N --steps K --warmup W`` (N>1 under torchrun, one
+rank per GPU).  Prints ONE JSON line on rank 0.
 
 * ``value``      device-timed throughput of the captured training step (forward +
                  backward + fused all-reduce/SGD/all-gather kernel), CUDA events,
@@ -14,6 +14,13 @@ torchrun, one rank per GPU).  Prints ONE JSON line on rank 0.
                  THIS process on THIS lease right before the shipyard arm, in two flavours (stock-eager, stock-tuned), each
                  device-timed and end to end with its own clocks; ``vs_stock_eager`` / ``vs_stock_tuned`` are value ratios.
 * ``collectives`` (N > 1) 256 MB all-reduce bus bandwidth and 8 B all-reduce latency, shipyard kernels vs NCCL, same run.
+* ``--dump-outputs DIR``  after the timed steps, rank 0 writes what the last captured
+                 step computed as DIR/<name>.npy: ``loss``, the model ``weights`` (bf16,
+                 as float32), rank 0's fp32 ``master_weights`` and the floating-point
+                 module ``buffers`` (BatchNorm running statistics).  Weight vectors over
+                 4 Mi elements are reduced to the same fixed, seeded sample of positions.
+                 Inputs and initial weights are seeded, so two builds can be compared
+                 output for output.
 * ``--impl reference``  the unmodified reference cannot be installed offline
                  (no setup.py/pyproject; imports azure.* at module load) -> prints
                  ``{"impl": "reference", "unavailable": ...}``.
@@ -47,7 +54,13 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-baseline", action="store_true", help="skip the same-run stock-PyTorch arms (bench/stock_baseline.py)")
     ap.add_argument("--no-coll", action="store_true", help="skip the same-run collective block (N > 1)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "shipyard":
+        ap.error("--dump-outputs needs --impl shipyard")
+    return args
 
 
 class ClockSampler:
@@ -176,6 +189,8 @@ def run_shipyard(args, rank, world, local):
     ms = timed(lambda i: tr.step(), args.steps, world, dev)
     clocks = sampler.stop() if rank == 0 else {}
     comm.check_status()
+    if args.dump_outputs and rank == 0:
+        _dump_outputs(args.dump_outputs, tr)
     loss_dev = float(tr.static_loss)
     # --- end-to-end through the public API: pinned uint8 -> H2D -> convert -> step -> loss D2H
     e2e = None
@@ -246,6 +261,32 @@ def run_shipyard(args, rank, world, local):
             out["collectives"] = {"error": f"{type(e).__name__}: {e}"[:200]}
     comm.close()
     return out
+
+
+DUMP_SAMPLE = 4 << 20          # elements kept of each weight vector: 2 x 16 MB of float32
+
+
+def _dump_outputs(out_dir: str, tr) -> None:
+    """Writes what the last training step left for the caller (see --dump-outputs) as float32 .npy files."""
+    import numpy as np
+    import torch
+    flat = tr.flat
+    total = flat.params.numel()
+    pos = None
+    if total > DUMP_SAMPLE:
+        pos = torch.randperm(total, generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+    lo, cnt = flat.shard
+    in_shard = torch.arange(lo, lo + cnt) if pos is None else pos[(pos >= lo) & (pos < lo + cnt)]
+    weights = flat.params.float().cpu()
+    arrays = {
+        "loss": tr.static_loss.detach().float().cpu().reshape(1),
+        "weights": weights if pos is None else weights[pos],
+        "master_weights": flat.master.float().cpu()[in_shard - lo],
+        "buffers": torch.cat([b.detach().float().cpu().reshape(-1) for b in tr.model.buffers() if b.is_floating_point()]),
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy().astype(np.float32))
 
 
 def _collective_block(comm, rank, world, dev) -> dict:

@@ -26,6 +26,21 @@ def pytest_collection_modifyitems(config, items):
             item.add_marker(pytest.mark.skip(reason="needs >= 2 GPUs"))
 
 
+@pytest.fixture(autouse=True)
+def _cpu_tests_see_no_gpu(request, monkeypatch):
+    """A test not marked `gpu` models a CPU-only box, where pools get virtual CPU-slot nodes (`cpu-<i>`).  On a machine with GPUs
+    the local backend would make one node per GPU and refuse a pool with more nodes than GPUs, so these tests see zero GPUs
+    whatever the machine has (the GPU probe honours SHIPYARD_FAKE_GPUS; a test may set its own count)."""
+    if "gpu" in request.keywords:
+        yield
+        return
+    from batch_shipyard_b200.pool import topology
+    monkeypatch.setenv("SHIPYARD_FAKE_GPUS", "0")
+    topology.probe(refresh=True)
+    yield
+    topology._CACHE = None                     # the next probe reads the real machine again
+
+
 @pytest.fixture(scope="session", autouse=True)
 def _native_executables():
     """Built artefacts are not in the history (see .gitignore); the libraries build themselves on first load (ops/*.py), the

@@ -1,20 +1,16 @@
-"""Option-by-option comparison of the click command tree with the reference's `shipyard.py` (read as text, never imported).
+"""Option-by-option comparison of the click command tree with the reference's `shipyard.py`.
 
-Skipped when the reference checkout is not mounted (e.g. on the GPU box)."""
+The reference's commands, their options, its SHIPYARD_* environment variables and the `--raw` capable commands of its usage guide
+are stored in tests/golden/reference/cli.json (Batch Shipyard 3.9.1, see make_golden.py there)."""
+import json
 import os
-import re
-
-def _read(path):
-    with open(path) as f:
-        return f.read()
-
 
 import click
-import pytest
 
 from batch_shipyard_b200 import cli
 
-REF = "/root/reference/shipyard.py"
+with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference", "cli.json")) as _f:
+    REF = json.load(_f)
 # options every command gets through shared decorators on both sides
 COMMON = {"--configdir", "--credentials", "--config", "--pool", "--jobs", "--fs", "--monitor", "--federation", "--slurm", "--raw", "--yes",
           "--verbose", "--show-config"}
@@ -33,16 +29,14 @@ def _ours():
     return out
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference checkout not mounted")
 def test_every_reference_option_exists_on_the_same_command():
-    src = _read(REF)
-    blocks = re.findall(r"@(\w+)\.command\('([\w-]+)'\)(.*?)\ndef (\w+)\(", src, flags=re.S)
+    blocks = REF["commands"]
     assert len(blocks) == 105
     ours = _ours()
     assert len(ours) == 105
     missing = []
-    for grp, name, decos, fn in blocks:
-        opts = set(re.findall(r"@click\.option\(\s*'(--[\w-]+)'", decos)) - COMMON
+    for grp, name, fn, ref_opts in blocks:
+        opts = set(ref_opts) - COMMON
         # the function name spells the command path: fed_jobs_del -> ("fed", "jobs", "del"); names keep their dashes
         # (sub-group commands drop the top group: nodes_count is `pool nodes count`, sas_create is `storage sas create`)
         joined = {k: "_".join(k).replace("-", "_") for k in ours}
@@ -55,15 +49,12 @@ def test_every_reference_option_exists_on_the_same_command():
     assert missing == [], missing
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/docs/20-batch-shipyard-usage.md"), reason="reference checkout not mounted")
 def test_raw_capable_commands_and_environment_variables_of_the_usage_guide_exist():
     """docs/20-batch-shipyard-usage.md lists the ~30 commands that support --raw and the SHIPYARD_* variables of the CLI."""
-    txt = _read("/root/reference/docs/20-batch-shipyard-usage.md")
-    block = txt[txt.index("The following commands support this option:"):txt.index("`--show-config` will output")]
-    listed = [tuple(m.split()) for m in re.findall(r"\* `([a-z \-]+)`", block)]
+    listed = [tuple(m.split()) for m in REF["raw_commands"]]
     assert len(listed) >= 30
     ours = _ours()
     assert [c for c in listed if c not in ours] == []
     src = open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "batch_shipyard_b200", "cli.py")).read()
-    env = set(re.findall(r"envvar='(SHIPYARD_[A-Z_]+)'", _read(REF)))
+    env = set(REF["envvars"])
     assert len(env) >= 20 and sorted(e for e in env if e not in src) == []

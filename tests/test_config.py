@@ -9,17 +9,15 @@ from batch_shipyard_b200.config import loader, settings as S
 from batch_shipyard_b200.config.schema import ConfigType, ValidationError, compile_schema, validate
 from batch_shipyard_b200.utils import util
 
-REF_TEMPLATES = "/root/reference/config_templates"
+REF_TEMPLATES = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference", "config_templates")   # Batch Shipyard 3.9.1
 
 
 @pytest.mark.parametrize("ct,name", [(ConfigType.Credentials, "credentials"), (ConfigType.Global, "config"), (ConfigType.Pool, "pool"),
                                      (ConfigType.Jobs, "jobs"), (ConfigType.RemoteFS, "fs"), (ConfigType.Monitor, "monitor"),
                                      (ConfigType.Federation, "federation"), (ConfigType.Slurm, "slurm")])
 def test_reference_templates_validate(ct, name):
-    p = os.path.join(REF_TEMPLATES, name + ".yaml")
-    if not os.path.exists(p):
-        pytest.skip("reference templates not mounted")
-    validate(ct, yaml.safe_load(open(p)))
+    with open(os.path.join(REF_TEMPLATES, name + ".yaml")) as f:
+        validate(ct, yaml.safe_load(f))
 
 
 def test_schema_strictness():

@@ -34,7 +34,7 @@ def test_multi_gpu_collectives(transport):
 
 
 @pytest.mark.multigpu
-def test_nccl_preload_shim_under_torch_distributed():
+def test_nccl_preload_shim_under_torch_distributed(tmp_path):
     """LD_PRELOAD the shim under a torchrun NCCL job: results stay correct and the collectives ran on our kernels."""
     _need_multi()
     import os
@@ -48,9 +48,7 @@ def test_nccl_preload_shim_under_torch_distributed():
     p = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={world}", "--master-addr", "127.0.0.1",
                         "--master-port", "29577", os.path.join(root, "tests", "_preload_worker.py")], env=env, stdout=subprocess.PIPE,
                        stderr=subprocess.STDOUT, text=True, timeout=600)
-    os.makedirs(os.path.join(root, "gpurun_out"), exist_ok=True)
-    with open(os.path.join(root, "gpurun_out", "preload_test.log"), "w") as f:
-        f.write(p.stdout)
+    (tmp_path / "preload_test.log").write_text(p.stdout)
     assert p.returncode == 0, p.stdout[-6000:]
     assert p.stdout.count("ok=True") == world
 

@@ -1,21 +1,18 @@
 """The full-document YAML examples in the reference's configuration guides (docs/11..18) validate against our schemas.
 
+The examples are stored under tests/golden/reference (guide_yaml_examples.json, taken from Batch Shipyard 3.9.1).
 Two examples contain typos that the reference's own schema rejects as well (`polling_interval.jobs` in the federation guide,
-`preempty_type` in the Slurm guide); those keys are removed before validation.  Skipped when the reference is not mounted."""
+`preempty_type` in the Slurm guide); those keys are removed before validation."""
+import json
 import os
-import re
-
-def _read(path):
-    with open(path) as f:
-        return f.read()
-
 
 import pytest
 import yaml
 
 from batch_shipyard_b200.config.schema import ConfigType, validate
 
-DOCS = "/root/reference/docs"
+with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference", "guide_yaml_examples.json")) as _f:
+    EXAMPLES = json.load(_f)
 CASES = [("11-batch-shipyard-configuration-credentials.md", ConfigType.Credentials, ("credentials",)),
          ("13-batch-shipyard-configuration-pool.md", ConfigType.Pool, ("pool_specification",)),
          ("14-batch-shipyard-configuration-jobs.md", ConfigType.Jobs, ("job_specifications",)),
@@ -33,12 +30,10 @@ def _strip_doc_typos(ct, data):
             part.pop("preempty_type", None)
 
 
-@pytest.mark.skipif(not os.path.isdir(DOCS), reason="reference checkout not mounted")
 @pytest.mark.parametrize("doc,ct,roots", CASES, ids=[c[0][:2] for c in CASES])
 def test_reference_guide_examples_validate(doc, ct, roots):
-    blocks = re.findall(r"```yaml\n(.*?)```", _read(os.path.join(DOCS, doc)), flags=re.S)
     n = 0
-    for b in blocks:
+    for b in EXAMPLES[doc]:
         try:
             data = yaml.safe_load(b)
         except yaml.YAMLError:
