@@ -199,6 +199,64 @@ def synthetic_cifar(n: int, seed: int, num_classes: int = 10, size: int = 32):
     return (x.clamp(0, 1) * 255).to(torch.uint8).permute(0, 2, 3, 1).contiguous(), y
 
 
+def _torchvision_name_map(model: ResNet) -> dict:
+    """torchvision resnet state-dict key -> (our tensor, kind) for every parameter and BN statistic of ``model``."""
+    out = {}
+
+    def cb(prefix_conv, prefix_bn, c: ConvBN):
+        out[prefix_conv + ".weight"] = c.weight
+        out[prefix_bn + ".weight"] = c.gamma
+        out[prefix_bn + ".bias"] = c.beta
+        out[prefix_bn + ".running_mean"] = c.running_mean
+        out[prefix_bn + ".running_var"] = c.running_var
+
+    cb("conv1", "bn1", model.stem)
+    # our blocks are one flat Sequential; torchvision groups them into layer1..layer4, and the first block of every stage is the one
+    # with a projection shortcut (the width changes by the expansion factor at every stage start)
+    layers = []
+    for b in model.blocks:
+        if not layers or b.down is not None:
+            layers.append([])
+        layers[-1].append(b)
+    for li, blocks in enumerate(layers):
+        for j, b in enumerate(blocks):
+            p = f"layer{li + 1}.{j}"
+            cb(p + ".conv1", p + ".bn1", b.c1)
+            cb(p + ".conv2", p + ".bn2", b.c2)
+            cb(p + ".conv3", p + ".bn3", b.c3)
+            if b.down is not None:
+                cb(p + ".downsample.0", p + ".downsample.1", b.down)
+    out["fc.weight"] = model.fc_weight
+    out["fc.bias"] = model.fc_bias
+    return out
+
+
+def load_torchvision_state_dict(model: ResNet, sd: dict) -> ResNet:
+    """Copy a torchvision ResNet (Bottleneck) state dict into ``model``: ``conv1`` / ``bn1``, ``layerX.Y.convZ`` / ``bnZ``,
+    ``layerX.Y.downsample.0`` / ``.1`` and ``fc``, running statistics included (``num_batches_tracked`` is ignored).
+
+    Raises ``KeyError`` listing the names on any unused key, missing key or shape mismatch, and changes nothing in that case.
+    Call it before building a trainer: ``FusedDataParallelTrainer`` takes its fp32 master copy of the weights at construction."""
+    names = _torchvision_name_map(model)
+    keys = {k for k in sd if not k.endswith("num_batches_tracked")}
+    unused = sorted(keys - set(names))
+    missing = sorted(set(names) - keys)
+    shape = sorted(k for k in keys & set(names) if tuple(sd[k].shape) != tuple(names[k].shape))
+    if unused or missing or shape:
+        parts = []
+        if unused:
+            parts.append("unused keys: " + ", ".join(unused))
+        if missing:
+            parts.append("missing keys: " + ", ".join(missing))
+        if shape:
+            parts.append("shape mismatch: " + ", ".join(f"{k} {tuple(sd[k].shape)} vs {tuple(names[k].shape)}" for k in shape))
+        raise KeyError("; ".join(parts))
+    with torch.no_grad():
+        for k, t in names.items():
+            t.copy_(sd[k].to(device=t.device, dtype=t.dtype))
+    return model
+
+
 def set_tc_gemm(m: nn.Module, flag: bool) -> None:
     for mod in m.modules():
         if hasattr(mod, "use_tc_gemm"):

@@ -90,6 +90,7 @@ def set_mode(mode: str) -> None:
     assert mode in ("auto", "tc", "cudnn")
     _MODE = mode
     _PLANS.clear()
+    _INFER_PLANS.clear()
 
 
 def set_halo(on: bool) -> None:
@@ -421,6 +422,77 @@ class _Conv(torch.autograd.Function):
             dw = _wgrad_tc(dy, x, w, stride, pad, _grad_view(ctx.w_ref), True,      # None when written into .grad in place
                            impl=plan.wgrad if plan.wgrad != "tc" else None)
         return dx, dw, None, None
+
+
+# ---- inference: convolution + folded BatchNorm (+ residual) (+ ReLU) ------------------------------------------------------------------
+# A table of its own, so the training plans (and bench.py's report of them) never change because an evaluation ran.  Two candidates
+# per shape: the own tcgen05 kernel with the affine epilogue (ops.gemm.conv_affine_nhwc), and cuDNN followed by ops.fused.bn_infer_apply.
+_INFER_PLANS: dict = {}
+
+
+@dataclass
+class InferPlan:
+    impl: str = "cudnn"       # "tc" (conv_affine_nhwc) | "cudnn" (F.conv2d + bn_infer_apply)
+    timings_us: Optional[dict] = None
+
+
+def infer_plan_table() -> dict:
+    return {"x".join(map(str, k)): asdict(v) for k, v in _INFER_PLANS.items()}
+
+
+def _infer_key(x, w, stride, residual, relu):
+    return _key(x, w, stride) + (int(residual), int(relu))
+
+
+def _infer_tc(x, w, scale, shift, stride, residual, relu):
+    return _gemm.conv_affine_nhwc(x, w, scale, shift, stride, residual=residual, relu=relu)
+
+
+def _infer_cudnn(x, w, scale, shift, stride, residual, relu):
+    from .fused import bn_infer_apply
+    y = F.conv2d(x, w, None, stride, w.shape[2] // 2)
+    if not y.is_contiguous(memory_format=torch.channels_last):
+        y = y.contiguous(memory_format=torch.channels_last)
+    return bn_infer_apply(y, scale, shift, residual, relu, out=y)
+
+
+def infer_plan_for(x: torch.Tensor, w: torch.Tensor, stride: int, residual: bool, relu: bool, use_tc: bool = True) -> InferPlan:
+    """The inference implementation of one layer shape: raced once (device-timed, outside any graph capture) in ``auto`` mode,
+    the own kernel wherever it applies in ``tc`` mode, cuDNN in ``cudnn`` mode or when ``use_tc`` (the layer's use_tc_gemm) is off."""
+    key = _infer_key(x, w, stride, residual, relu)
+    p = _INFER_PLANS.get(key)
+    if p is not None:
+        return p
+    ok = use_tc and _gemm.conv_affine_ok(x, w, stride)
+    if _MODE == "cudnn" or not ok:
+        p = InferPlan("cudnn", {})
+    elif _MODE == "tc":
+        p = InferPlan("tc", {})
+    else:
+        if torch.cuda.is_current_stream_capturing():
+            raise RuntimeError("infer_plan_for: shape %s was not raced before graph capture" % (key,))
+        cout = w.shape[0]
+        scale = torch.rand(cout, device=x.device) + 0.5
+        shift = torch.randn(cout, device=x.device)
+        n, _, h, wd = x.shape
+        k = w.shape[2]
+        pq = ((h + 2 * (k // 2) - k) // stride + 1, (wd + 2 * (k // 2) - k) // stride + 1)
+        r = torch.randn((n, cout) + pq, device=x.device).to(torch.bfloat16).contiguous(memory_format=torch.channels_last) if residual else None
+        xd, wd_ = x.detach(), w.detach()
+        with torch.no_grad():
+            t = {"fprop_cudnn": _time(lambda: _infer_cudnn(xd, wd_, scale, shift, stride, r, relu)),
+                 "fprop_tc": _time(lambda: _infer_tc(xd, wd_, scale, shift, stride, r, relu))}
+        p = InferPlan(_pick(t, "fprop_").split("_")[1], {k_: round(v, 1) for k_, v in t.items()})
+    _INFER_PLANS[key] = p
+    return p
+
+
+def conv_bn_infer(x: torch.Tensor, w: torch.Tensor, scale: torch.Tensor, shift: torch.Tensor, stride: int = 1,
+                  residual: Optional[torch.Tensor] = None, relu: bool = True, use_tc: bool = True) -> torch.Tensor:
+    """act(conv2d(x, w) * scale + shift (+ residual)) through the layer shape's inference plan (channels_last bf16)."""
+    plan = infer_plan_for(x, w, stride, residual is not None, relu, use_tc)
+    fn = _infer_tc if plan.impl == "tc" else _infer_cudnn
+    return fn(x, w, scale, shift, stride, residual, relu)
 
 
 def conv_bn_input(x: torch.Tensor, w: torch.Tensor, stride: int = 1):

@@ -76,6 +76,8 @@ def _bind_bn(lib):
     lib.sy_ops_maxpool3x3s2_fwd.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp]
     lib.sy_ops_maxpool3x3s2_bwd.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp]
     lib.sy_ops_u8_to_s2d_norm.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_float), vp]
+    lib.sy_ops_bn_fold.argtypes = [vp, C.c_int, vp]
+    lib.sy_ops_bn_infer_apply.argtypes = [vp, vp, vp, fp, fp, C.c_long, C.c_int, C.c_int, vp]
     lib._bn_bound = True
 
 
@@ -279,6 +281,85 @@ class _MaxPool3x3s2(torch.autograd.Function):
 
 def maxpool3x3s2(x: torch.Tensor) -> torch.Tensor:
     return _MaxPool3x3s2.apply(x)
+
+
+def maxpool3x3s2_infer(x: torch.Tensor) -> torch.Tensor:
+    """Inference max-pool 3x3/s2/p1 on channels_last bf16 (no arg-max codes: nothing is kept for a backward pass)."""
+    lib = load(); _bind_bn(lib)
+    assert x.is_cuda and x.dtype == torch.bfloat16 and _is_nhwc(x) and x.shape[1] % 8 == 0
+    n, c, h, w = x.shape
+    oh, ow = (h + 2 - 3) // 2 + 1, (w + 2 - 3) // 2 + 1
+    y = torch.empty((n, oh, ow, c), dtype=x.dtype, device=x.device).permute(0, 3, 1, 2)
+    rc = lib.sy_ops_maxpool3x3s2_fwd(_ptr(x), _ptr(y), None, n, h, w, c, _stream(x))
+    if rc != 0:
+        raise RuntimeError(f"maxpool (inference) failed ({rc})")
+    return y
+
+
+# ---------------------------------------------------------------------------
+# inference BatchNorm: folded per-channel affine maps
+# ---------------------------------------------------------------------------
+def bn_fold_reference(gamma, beta, running_mean, running_var, eps=1e-5):
+    """(scale, shift) in fp32 with BN_eval(x) = x * scale + shift: the formula the fold kernel computes."""
+    scale = gamma.float() * torch.rsqrt(running_var.float() + eps)
+    return scale, beta.float() - running_mean.float() * scale
+
+
+class BnFoldTable:
+    """Device table for ``bn_fold``: one 64-byte entry {gamma, beta, running_mean, running_var, scale_out, shift_out, C, eps} per BN
+    layer, and the fp32 scale / shift outputs (every layer's slice 32-byte aligned for the 16-byte vector loads of the consumers).
+
+    The entries hold raw pointers to the parameters and statistics: the table stays valid while those tensors keep their storage."""
+
+    def __init__(self, layers, device):
+        """layers: list of (gamma bf16[C], beta bf16[C], running_mean fp32[C], running_var fp32[C], eps)."""
+        import struct
+        offs, total = [], 0
+        for g, b, m, v, _ in layers:
+            c = g.numel()
+            assert g.dtype == torch.bfloat16 and b.dtype == torch.bfloat16, "bn_fold: gamma / beta must be bf16"
+            assert m.dtype == torch.float32 and v.dtype == torch.float32, "bn_fold: running statistics must be fp32"
+            assert all(t.is_cuda and t.is_contiguous() and t.numel() == c for t in (g, b, m, v))
+            offs.append(total)
+            total += (c + 7) // 8 * 8
+        self.buf = torch.zeros(2, max(total, 8), dtype=torch.float32, device=device)
+        self.scale = [self.buf[0, o:o + g.numel()] for o, (g, *_r) in zip(offs, layers)]
+        self.shift = [self.buf[1, o:o + g.numel()] for o, (g, *_r) in zip(offs, layers)]
+        words = []
+        for (g, b, m, v, eps), sc, sh in zip(layers, self.scale, self.shift):
+            eps_bits = struct.unpack("<I", struct.pack("<f", float(eps)))[0]
+            words += [g.data_ptr(), b.data_ptr(), m.data_ptr(), v.data_ptr(), sc.data_ptr(), sh.data_ptr(), g.numel(), eps_bits]
+        self.table = torch.tensor(words, dtype=torch.int64).to(device)
+        self.n_layers = len(layers)
+        self._keep = layers                       # the pointed-to tensors must outlive the table
+
+
+def bn_fold(table: BnFoldTable) -> None:
+    """scale = gamma * rsqrt(running_var + eps), shift = beta - running_mean * scale for every layer of ``table``: ONE launch."""
+    lib = load(); _bind_bn(lib)
+    rc = lib.sy_ops_bn_fold(_ptr(table.table), table.n_layers, _stream(table.table))
+    if rc != 0:
+        raise RuntimeError(f"bn_fold failed ({rc})")
+
+
+def bn_infer_apply(x: torch.Tensor, scale: torch.Tensor, shift: torch.Tensor, residual=None, relu: bool = True,
+                   out=None) -> torch.Tensor:
+    """out = act(x * scale + shift (+ residual)) on channels_last bf16 (inference BatchNorm of a layer whose convolution has no
+    fused epilogue).  ``out`` may be ``x`` (in place)."""
+    lib = load(); _bind_bn(lib)
+    assert x.is_cuda and x.dtype == torch.bfloat16 and _is_nhwc(x), "bn_infer_apply wants channels_last bf16"
+    n, c, h, w = x.shape
+    assert c % 8 == 0, "bn_infer_apply: channels % 8"
+    assert scale.dtype == torch.float32 and shift.dtype == torch.float32 and scale.numel() == c and shift.numel() == c
+    if residual is not None:
+        assert residual.shape == x.shape and residual.dtype == x.dtype and _is_nhwc(residual)
+    out = torch.empty_like(x) if out is None else out
+    assert out.shape == x.shape and _is_nhwc(out)
+    rc = lib.sy_ops_bn_infer_apply(_ptr(x), _ptr(residual), _ptr(out), _ptr(scale), _ptr(shift), n * h * w, c, 1 if relu else 0,
+                                   _stream(x))
+    if rc != 0:
+        raise RuntimeError(f"bn_infer_apply failed ({rc})")
+    return out
 
 
 def u8_to_s2d_norm(src_u8: torch.Tensor, dst: torch.Tensor, mean=IMAGENET_MEAN, std=IMAGENET_STD) -> torch.Tensor:

@@ -55,6 +55,10 @@ def load() -> C.CDLL:
         lib.sy_conv3x3_wgrad_halo.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p] + [C.c_int] * 5 + [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]
         lib.sy_gemm_bf16_nn_scatter2.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p] + [C.c_int] * 7 + [C.c_void_p]
         lib.sy_stem_s2d_fprop.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p]
+        lib.sy_gemm_bf16_tn_affine.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p] + [C.c_int] * 6 + [C.c_void_p, C.c_void_p, C.c_void_p] + \
+            [C.c_int] * 4 + [C.c_void_p]
+        lib.sy_conv_bf16_nhwc_affine.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p] + [C.c_int] * 9 + [C.c_void_p, C.c_void_p, C.c_void_p] + \
+            [C.c_int] * 3 + [C.c_void_p]
         lib.sy_stem_s2d_wgrad.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
                                           C.c_void_p]
         _LIB = lib
@@ -651,3 +655,55 @@ class _StemS2D(torch.autograd.Function):
 def stem_conv_s2d(x: torch.Tensor, w2: torch.Tensor, want_stats: bool = True):
     """(y, stats) of the s2d stem convolution; stats is None when not requested."""
     return _StemS2D.apply(x, w2, want_stats)
+
+
+# ---- inference: BatchNorm folded into the GEMM / convolution epilogue ------------------------------------------------------------
+def conv_affine_ok(x: torch.Tensor, w: torch.Tensor, stride: int) -> bool:
+    """Shapes ``conv_affine_nhwc`` accepts: 1x1 / stride 1 as a GEMM (channels % 8), anything else through the im2col kernel
+    (input channels % 64, output channels % 8, N*P*Q % 128)."""
+    if not (x.is_cuda and x.dtype == torch.bfloat16 and w.dtype == torch.bfloat16):
+        return False
+    cin, cout, k = x.shape[1], w.shape[0], w.shape[2]
+    if k == 1 and stride == 1:
+        return cin % 8 == 0 and cout % 8 == 0
+    return conv_supported(x, w, stride, k // 2)
+
+
+def conv_affine_nhwc(x: torch.Tensor, w: torch.Tensor, scale: torch.Tensor, shift: torch.Tensor, stride: int = 1,
+                     residual: Optional[torch.Tensor] = None, relu: bool = True, block_n: int = 0, max_ctas: int = 0) -> torch.Tensor:
+    """y = act(conv2d(x, w, stride, 'same') * scale + shift (+ residual)) for channels_last bf16 x[N,Cin,H,W], w[Cout,Cin,K,K] (stored
+    KRSC), fp32 scale / shift [Cout], optional channels_last bf16 residual shaped like y: the inference form of conv + BatchNorm
+    (+ residual add) (+ ReLU) in ONE tcgen05 kernel, accumulator scaled in fp32 and rounded to bf16 once.  1x1 / stride 1 runs as the
+    GEMM, everything else as the TMA-im2col convolution.  Returns channels_last y."""
+    n, cin, h, wd = x.shape
+    cout, _, r, s = w.shape
+    pad = r // 2
+    p, q = (h + 2 * pad - r) // stride + 1, (wd + 2 * pad - s) // stride + 1
+    assert x.is_cuda and x.dtype == torch.bfloat16 and w.dtype == torch.bfloat16 and w.shape[1] == cin and r == s
+    assert scale.dtype == torch.float32 and shift.dtype == torch.float32 and scale.numel() == cout and shift.numel() == cout
+    assert scale.is_contiguous() and shift.is_contiguous()
+    assert cout % 8 == 0, "conv_affine_nhwc: output channels % 8"
+    xs, ws = _nhwc_storage(x), _nhwc_storage(w)
+    rs = None
+    if residual is not None:
+        assert tuple(residual.shape) == (n, cout, p, q) and residual.dtype == torch.bfloat16
+        rs = _nhwc_storage(residual)
+    y = torch.empty((n, p, q, cout), dtype=torch.bfloat16, device=x.device)
+    lib = load()
+    stream = C.c_void_p(torch.cuda.current_stream(x.device).cuda_stream)
+    rptr = C.c_void_p(rs.data_ptr() if rs is not None else 0)
+    if r == 1 and stride == 1:
+        assert cin % 8 == 0, "1x1 GEMM: input channels % 8"
+        rc = lib.sy_gemm_bf16_tn_affine(C.c_void_p(xs.data_ptr()), C.c_void_p(ws.data_ptr()), C.c_void_p(y.data_ptr()), n * h * wd, cout, cin,
+                                        cin, cin, cout, C.c_void_p(scale.data_ptr()), C.c_void_p(shift.data_ptr()), rptr, cout,
+                                        1 if relu else 0, block_n, max_ctas, stream)
+        if rc != 0:
+            raise RuntimeError(f"sy_gemm_bf16_tn_affine failed ({rc}): {lib.sy_gemm_last_error().decode()}")
+    else:
+        assert conv_supported(x, w, stride, pad), "conv_affine_nhwc: input channels % 64 and N*P*Q % 128 for the im2col kernel"
+        rc = lib.sy_conv_bf16_nhwc_affine(C.c_void_p(xs.data_ptr()), C.c_void_p(ws.data_ptr()), C.c_void_p(y.data_ptr()), n, h, wd, cin, cout,
+                                          r, s, pad, stride, C.c_void_p(scale.data_ptr()), C.c_void_p(shift.data_ptr()), rptr,
+                                          1 if relu else 0, block_n, max_ctas, stream)
+        if rc != 0:
+            raise RuntimeError(f"sy_conv_bf16_nhwc_affine failed ({rc}): {lib.sy_gemm_last_error().decode()}")
+    return y.permute(0, 3, 1, 2)

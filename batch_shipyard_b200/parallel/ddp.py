@@ -208,6 +208,67 @@ class FusedDataParallelTrainer:
     def set_lr(self, lr: float) -> None:
         self.hyper[0:1].fill_(lr)
 
+    # -- evaluation --------------------------------------------------------------
+    def evaluate(self, images_u8: torch.Tensor, labels: torch.Tensor, batch: Optional[int] = None) -> dict:
+        """Held-out metrics of this rank's shard, summed over all ranks: {"count", "loss" (summed cross-entropy), "top1", "top5"}.
+
+        ResNet models on a GPU run on ``parallel.infer.ResNetInference`` (built once per batch size and cached); any other model, and
+        every CPU run, uses the module's own eval forward under ``no_grad`` on the input conversion training uses, then restores the
+        module's train/eval mode.  No training state changes: flat parameters and gradients, fp32 master, momentum, running
+        statistics, the static step inputs and the captured step graph stay as they were, so this may run between steps.
+        Every rank must call it (the per-rank sums meet in one all-reduce)."""
+        from ..models.resnet import ResNet, ResNetCifar
+        n_total = int(images_u8.shape[0])
+        bs = int(batch or self.batch_shape[0])
+        sums = torch.zeros(4, dtype=torch.float64)
+        use_engine = self.is_cuda and isinstance(self.model, (ResNet, ResNetCifar))
+        eng = None
+        if use_engine and n_total > 0:
+            engines = self.__dict__.setdefault("_engines", {})
+            eng = engines.get(bs)
+            if eng is None:
+                from .infer import ResNetInference
+                eng = engines[bs] = ResNetInference(self.model, bs, image_size=int(images_u8.shape[1]))
+        for i in range(0, n_total, bs):
+            x = images_u8[i:i + bs].to(self.dev, non_blocking=True)
+            y = labels[i:i + bs].to(self.dev, non_blocking=True)
+            logits = eng(x) if eng is not None else self._eval_forward(x)
+            logits = logits.float()
+            k = min(5, logits.shape[1])
+            top = logits.topk(k, dim=1).indices
+            hit = top == y.view(-1, 1)
+            sums += torch.tensor([float(y.numel()), float(F.cross_entropy(logits, y, reduction="sum")),
+                                  float(hit[:, 0].sum()), float(hit.any(dim=1).sum())], dtype=torch.float64)
+        buf = self.__dict__.get("_eval_sym")
+        if buf is None:
+            buf = self._eval_sym = self.comm.alloc(4, torch.float64)       # symmetric: the same code runs on every transport
+        buf.copy_(sums.to(buf.device))
+        self.comm.all_reduce(buf)
+        if self.is_cuda:
+            torch.cuda.synchronize(self.dev)
+        out = buf.cpu().tolist()
+        return {"count": int(round(out[0])), "loss": out[1], "top1": int(round(out[2])), "top5": int(round(out[3]))}
+
+    def _eval_forward(self, images_u8: torch.Tensor) -> torch.Tensor:
+        """The module's own eval forward on the conversion training uses (not a hot path)."""
+        n, h, w, c = images_u8.shape
+        if self.is_cuda:
+            if self.s2d:
+                xs = torch.empty((n, h // 2 + 3, w // 2 + 3, 16), dtype=torch.bfloat16, device=self.dev)
+                _fused.u8_to_s2d_norm(images_u8, xs)
+            else:
+                xs = torch.empty((n, h, w, c), dtype=torch.bfloat16, device=self.dev)
+                _fused.u8_to_bf16_norm(images_u8, xs)
+        else:
+            xs = images_u8.to(torch.float32) / 255.0
+        was_training = self.model.training
+        self.model.eval()
+        try:
+            with torch.no_grad():
+                return self.model(xs.permute(0, 3, 1, 2))
+        finally:
+            self.model.train(was_training)
+
     # -- end-to-end input path -------------------------------------------------
     def make_stager(self, depth: int = 2) -> "InputStager":
         self._stager = InputStager(self, depth)

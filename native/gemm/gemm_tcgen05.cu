@@ -240,12 +240,25 @@ template <int BN> struct Cfg {
 // kEpiAlt (BN = 64, with kDirect): a 64-column tile has one epilogue chunk, so warpgroup g drains accumulator stage g (alternate
 // tiles) instead of group 1 idling — same schedule as conv3x3_halo_kernel's kEpiAlt.  [numerics verified on hardware in round 2; selected with
 // SHIPYARD_GEMM_DIRECT_STORE=1 SHIPYARD_GEMM_EPI_ALT=1]
-template <int BN, bool kStats, bool kBias, bool kBMN = false, bool kConv = false, bool kDirect = false, bool kEpiAlt = false>
+// Folded-BatchNorm epilogue (kAffine, inference): out[m, n] = act(acc[m, n] * scale[n] + shift[n] (+ residual[m, n])), all in fp32 on
+// the accumulator and rounded to bf16 once.  The residual (bf16, the output's NHWC layout, row pitch ldr) is read by the thread that owns
+// the output row, 16 bytes per load, before it waits for the accumulator.  Runs with the st.global store phase (kDirect).
+struct EpiAffine {
+  const float* scale;                 // [N] fp32, 16-byte aligned
+  const float* shift;                 // [N] fp32, 16-byte aligned
+  const __nv_bfloat16* residual;      // [M, ldr] or null; never the output itself
+  int ldr;
+  int relu;
+};
+
+template <int BN, bool kStats, bool kBias, bool kBMN = false, bool kConv = false, bool kDirect = false, bool kEpiAlt = false,
+          bool kAffine = false>
 __global__ void __launch_bounds__(kThreadsTN, 1)
 gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                     const __grid_constant__ CUtensorMap tmap_c, int M, int N, int K,
                     const __nv_bfloat16* __restrict__ bias, float* __restrict__ stats, const ConvGeom geom,
-                    __nv_bfloat16* __restrict__ c_ptr = nullptr, int ldc = 0) {
+                    __nv_bfloat16* __restrict__ c_ptr = nullptr, int ldc = 0, const EpiAffine aff = EpiAffine{}) {
+  static_assert(!kAffine || (kDirect && !kStats && !kBias && !kBMN && !kEpiAlt), "kAffine: plain forward GEMM / conv with the st.global epilogue");
   using C = Cfg<BN>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -402,6 +415,15 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
         for (int ci = 0; ci < kMyChunks; ++ci) {
           const int c = cg + ci * kEpiGroups;
           if (c >= kChunks) break;
+          uint4 rsd[8];                     // kAffine: this row's 64 residual columns, loaded while the TMEM read is in flight
+          if constexpr (kAffine) {
+            const int mrow = m_blk * BM + row, c0 = n_blk * BN + c * kEpiChunk;
+#pragma unroll
+            for (int q = 0; q < 8; ++q)
+              rsd[q] = (aff.residual && mrow < M && c0 + q * 8 < N)
+                           ? __ldg(reinterpret_cast<const uint4*>(aff.residual + (size_t)mrow * (size_t)aff.ldr + c0 + q * 8))
+                           : make_uint4(0u, 0u, 0u, 0u);
+          }
           tmem_ld_wait();
           const bool last = c + kEpiGroups >= kChunks;
           if (last) {                       // this group's part of the accumulator is in registers: hand it back early
@@ -419,7 +441,24 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
 #pragma unroll
               for (int i = 0; i < 8; ++i) { const int col = n0 + q * 8 + i; f[i] += col < N ? __bfloat162float(bias[col]) : 0.f; }
             }
-            w[q] = make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
+            if constexpr (kAffine) {        // N % 8 == 0: a 16-byte piece is wholly inside or wholly past the last column
+              if (n0 + q * 8 < N) {
+                const float4 s0 = __ldg(reinterpret_cast<const float4*>(aff.scale + n0 + q * 8));
+                const float4 s1 = __ldg(reinterpret_cast<const float4*>(aff.scale + n0 + q * 8 + 4));
+                const float4 t0 = __ldg(reinterpret_cast<const float4*>(aff.shift + n0 + q * 8));
+                const float4 t1 = __ldg(reinterpret_cast<const float4*>(aff.shift + n0 + q * 8 + 4));
+                const float s[8] = {s0.x, s0.y, s0.z, s0.w, s1.x, s1.y, s1.z, s1.w};
+                const float t[8] = {t0.x, t0.y, t0.z, t0.w, t1.x, t1.y, t1.z, t1.w};
+                const uint32_t rw[4] = {rsd[q].x, rsd[q].y, rsd[q].z, rsd[q].w};
+#pragma unroll
+                for (int i = 0; i < 8; ++i) {
+                  const float r = (i & 1) ? __uint_as_float(rw[i >> 1] & 0xffff0000u) : __uint_as_float(rw[i >> 1] << 16);
+                  f[i] = fmaf(f[i], s[i], t[i]) + r;
+                  if (aff.relu) f[i] = fmaxf(f[i], 0.f);
+                }
+              }
+            }
+            w[q] =make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
           }
           if (!last) {                      // prefetch this group's next chunk; its latency hides behind the store phase below
             tmem_ld32(tbase + (c + kEpiGroups) * kEpiChunk, v[0]);
@@ -1440,7 +1479,7 @@ int launch_conv(const void* act, const void* wgt, void* out, int Nb, int H, int 
   auto go = [&](auto kern) -> int {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::kSmemBytes);
     if (e != cudaSuccess) { snprintf(g_err, sizeof g_err, "smem attribute: %s", cudaGetErrorString(e)); return 4; }
-    kern<<<grid, kThreadsTN, C::kSmemBytes, s>>>(ta, tb, tc, M, N, K, (const __nv_bfloat16*)nullptr, stats, g, (__nv_bfloat16*)out, N);
+    kern<<<grid, kThreadsTN, C::kSmemBytes, s>>>(ta, tb, tc, M, N, K, (const __nv_bfloat16*)nullptr, stats, g, (__nv_bfloat16*)out, N, EpiAffine{});
     e = cudaGetLastError();
     if (e != cudaSuccess) { snprintf(g_err, sizeof g_err, "launch: %s", cudaGetErrorString(e)); return 5; }
     g_launches.fetch_add(1);
@@ -1471,7 +1510,8 @@ int launch(const void* A, const void* B, void* Cc, int M, int N, int K, int lda,
   auto go = [&](auto kern) -> int {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::kSmemBytes);
     if (e != cudaSuccess) { snprintf(g_err, sizeof g_err, "smem attribute: %s", cudaGetErrorString(e)); return 4; }
-    kern<<<grid, kThreadsTN, C::kSmemBytes, s>>>(ta, tb, tc, M, N, K, (const __nv_bfloat16*)bias, stats, ConvGeom{}, (__nv_bfloat16*)Cc, ldc);
+    kern<<<grid, kThreadsTN, C::kSmemBytes, s>>>(ta, tb, tc, M, N, K, (const __nv_bfloat16*)bias, stats, ConvGeom{}, (__nv_bfloat16*)Cc, ldc,
+                                                 EpiAffine{});
     e = cudaGetLastError();
     if (e != cudaSuccess) { snprintf(g_err, sizeof g_err, "launch: %s", cudaGetErrorString(e)); return 5; }
     g_launches.fetch_add(1);
@@ -1495,6 +1535,44 @@ int launch(const void* A, const void* B, void* Cc, int M, int N, int K, int lda,
   if (stats) return direct ? go(gemm_bf16_tn_kernel<BN, true, false, false, false, true>) : go(gemm_bf16_tn_kernel<BN, true, false>);
   if (bias) return go(gemm_bf16_tn_kernel<BN, false, true>);
   return direct ? go(gemm_bf16_tn_kernel<BN, false, false, false, false, true>) : go(gemm_bf16_tn_kernel<BN, false, false>);
+}
+
+// Folded-BN epilogue launches (kAffine): the plain GEMM (conv == false: A [M, K] row-major) or the TMA-im2col convolution.
+template <int BN>
+int launch_affine(bool conv, const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc, int M, int N, int K, const ConvGeom& g,
+                  void* out, int ldc, const EpiAffine& aff, int max_ctas, cudaStream_t s) {
+  using C = Cfg<BN>;
+  int dev = 0, sms = 148;
+  cudaGetDevice(&dev); cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int tiles = ((M + BM - 1) / BM) * ((N + BN - 1) / BN);
+  int grid = tiles < sms ? tiles : sms;
+  if (max_ctas > 0 && grid > max_ctas) grid = max_ctas;
+  auto go = [&](auto kern) -> int {
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::kSmemBytes);
+    if (e != cudaSuccess) { snprintf(g_err, sizeof g_err, "smem attribute: %s", cudaGetErrorString(e)); return 4; }
+    kern<<<grid, kThreadsTN, C::kSmemBytes, s>>>(ta, tb, tc, M, N, K, (const __nv_bfloat16*)nullptr, (float*)nullptr, g, (__nv_bfloat16*)out,
+                                                 ldc, aff);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) { snprintf(g_err, sizeof g_err, "launch: %s", cudaGetErrorString(e)); return 5; }
+    g_launches.fetch_add(1);
+    return 0;
+  };
+  return conv ? go(gemm_bf16_tn_kernel<BN, false, false, false, true, true, false, true>)
+              : go(gemm_bf16_tn_kernel<BN, false, false, false, false, true, false, true>);
+}
+
+// Shared argument checks of the two affine entry points: N % 8 (whole 16-byte pieces), aligned scale / shift / residual, and an output
+// that does not overlap the residual (a row's residual would be overwritten by another CTA before it is read).
+bool affine_args_ok(const void* out, long out_rows, int ldc, const float* scale, const float* shift, const void* residual, int ldr, int N) {
+  if (N % 8 || !scale || !shift || (((uintptr_t)scale | (uintptr_t)shift | (uintptr_t)residual) & 15) || (residual && (ldr & 7))) {
+    snprintf(g_err, sizeof g_err, "affine epilogue: N %% 8, 16-byte aligned scale / shift / residual, residual pitch %% 8"); return false;
+  }
+  if (residual) {
+    const uintptr_t o0 = (uintptr_t)out, o1 = o0 + (uintptr_t)out_rows * ldc * 2;
+    const uintptr_t r0 = (uintptr_t)residual, r1 = r0 + (uintptr_t)out_rows * ldr * 2;
+    if (o0 < r1 && r0 < o1) { snprintf(g_err, sizeof g_err, "affine epilogue: out must not alias residual"); return false; }
+  }
+  return true;
 }
 
 }  // namespace
@@ -1641,6 +1719,65 @@ extern "C" int sy_conv_bf16_nhwc(const void* act, const void* wgt, void* out, in
   return 1;
 }
 
+// Inference GEMM with BatchNorm folded into the epilogue (1x1 / stride-1 convolution on NHWC activations):
+//   C[m, n] = act(sum_k A[m, k] * B[n, k] * scale[n] + shift[n] (+ residual[m * ldr + n]))
+// act = ReLU when relu != 0, else identity; scale / shift fp32[N]; residual bf16 or null, and it must not overlap C.
+// Requirements: those of sy_gemm_bf16_tn, N %% 8 == 0, scale / shift / residual 16-byte aligned, ldr %% 8 == 0.  block_n 64, 128 or 256.
+extern "C" int sy_gemm_bf16_tn_affine(const void* A, const void* B, void* C, int M, int N, int K, int lda, int ldb, int ldc,
+                                      const float* scale, const float* shift, const void* residual, int ldr, int relu, int block_n,
+                                      int max_ctas, void* stream) {
+  if (M <= 0 || N <= 0 || K <= 0) return 0;
+  if ((lda | ldb | ldc) & 7 || ((uintptr_t)A | (uintptr_t)B | (uintptr_t)C) & 15) {
+    snprintf(g_err, sizeof g_err, "alignment: pointers must be 16B aligned and leading dimensions multiples of 8");
+    return 1;
+  }
+  if (!affine_args_ok(C, M, ldc, scale, shift, residual, ldr, N)) return 1;
+  if (!load_encode()) { snprintf(g_err, sizeof g_err, "cuTensorMapEncodeTiled unavailable (no driver?)"); return 6; }
+  if (block_n <= 0) block_n = N > 128 ? 256 : (N > 64 ? 128 : 64);
+  CUtensorMap ta, tb, tc;
+  if (!make_map(&ta, A, K, M, lda, BK, BM) || !make_map(&tc, C, N, M, ldc, kEpiChunk, BM)) return 3;
+  const EpiAffine aff{scale, shift, (const __nv_bfloat16*)residual, ldr, relu ? 1 : 0};
+  const ConvGeom g{};
+  cudaStream_t s = (cudaStream_t)stream;
+  switch (block_n) {
+    case 64: if (!make_map(&tb, B, K, N, ldb, BK, 64)) return 3; return launch_affine<64>(false, ta, tb, tc, M, N, K, g, C, ldc, aff, max_ctas, s);
+    case 128: if (!make_map(&tb, B, K, N, ldb, BK, 128)) return 3; return launch_affine<128>(false, ta, tb, tc, M, N, K, g, C, ldc, aff, max_ctas, s);
+    case 256: if (!make_map(&tb, B, K, N, ldb, BK, 256)) return 3; return launch_affine<256>(false, ta, tb, tc, M, N, K, g, C, ldc, aff, max_ctas, s);
+  }
+  snprintf(g_err, sizeof g_err, "block_n must be 64, 128 or 256");
+  return 1;
+}
+
+// Inference convolution with BatchNorm folded into the epilogue (TMA im2col implicit GEMM, 1-CTA):
+//   out[N,P,Q,c_out] = act(conv(act_in[N,H,W,c_act], wgt[c_out,R,S,c_act]) * scale + shift (+ residual[N,P,Q,c_out]))
+// Requirements: those of sy_conv_bf16_nhwc (c_act %% 64, c_out %% 8, N*P*Q %% 128), scale / shift / residual 16-byte aligned,
+// residual dense NHWC like `out` and not overlapping it.
+extern "C" int sy_conv_bf16_nhwc_affine(const void* act, const void* wgt, void* out, int Nb, int H, int W, int c_act, int c_out, int R, int S,
+                                        int pad, int stride, const float* scale, const float* shift, const void* residual, int relu,
+                                        int block_n, int max_ctas, void* stream) {
+  if (c_act % 64 || c_out % 8 || ((uintptr_t)act | (uintptr_t)wgt | (uintptr_t)out) & 15) {
+    snprintf(g_err, sizeof g_err, "conv: act channels %% 64, out channels %% 8, 16B aligned tensors"); return 1;
+  }
+  const int P = (H + 2 * pad - R) / stride + 1, Q = (W + 2 * pad - S) / stride + 1;
+  if (((long)Nb * P * Q) % BM) { snprintf(g_err, sizeof g_err, "conv: N*P*Q must be a multiple of 128"); return 1; }
+  const int M = Nb * P * Q, N = c_out, K = R * S * c_act;
+  if (!affine_args_ok(out, M, N, scale, shift, residual, N, N)) return 1;
+  if (!load_encode() || !load_encode_im2col()) { snprintf(g_err, sizeof g_err, "cuTensorMapEncode* unavailable (no driver?)"); return 6; }
+  if (block_n <= 0) block_n = c_out > 128 ? 256 : (c_out > 64 ? 128 : 64);
+  CUtensorMap ta, tb, tc;
+  if (!make_im2col_map(&ta, act, Nb, H, W, c_act, R, S, pad, stride, BM) || !make_map(&tc, out, N, M, N, kEpiChunk, BM)) return 3;
+  const EpiAffine aff{scale, shift, (const __nv_bfloat16*)residual, N, relu ? 1 : 0};
+  const ConvGeom g{P, Q, S, R * S, c_act / 64, stride, -pad, 0};
+  cudaStream_t s = (cudaStream_t)stream;
+  switch (block_n) {
+    case 64: if (!make_map(&tb, wgt, K, N, K, BK, 64)) return 3; return launch_affine<64>(true, ta, tb, tc, M, N, K, g, out, N, aff, max_ctas, s);
+    case 128: if (!make_map(&tb, wgt, K, N, K, BK, 128)) return 3; return launch_affine<128>(true, ta, tb, tc, M, N, K, g, out, N, aff, max_ctas, s);
+    case 256: if (!make_map(&tb, wgt, K, N, K, BK, 256)) return 3; return launch_affine<256>(true, ta, tb, tc, M, N, K, g, out, N, aff, max_ctas, s);
+  }
+  snprintf(g_err, sizeof g_err, "block_n must be 64, 128 or 256");
+  return 1;
+}
+
 // Convolution weight gradient: dW[Cout][R][S][Cin] (+)= sum over output pixels of dY[pix][Cout] * im2col(x)[pix][(r,s,Cin)].
 // One split-K launch covers every filter tap (work item = (tap, tile, K-split)).  ws: float[R*S*Cin*Cout], tickets:
 // int[R*S*tiles]; both zero on entry and on exit.  Requirements: Cin %% 64, Cout %% 8, N*P*Q %% 128.
@@ -1778,7 +1915,7 @@ extern "C" int sy_gemm_bf16_nn_scatter2(const void* dY, const void* W, void* dX,
     if (e != cudaSuccess) { snprintf(g_err, sizeof g_err, "smem attribute: %s", cudaGetErrorString(e)); return 4; }
     ConvGeom g{P, Q, 1, 1, 0, 2, 0, 0};
     kern<<<grid, kThreadsTN, C::kSmemBytes, (cudaStream_t)stream>>>(ta, tb, tc, M, N, K, (const __nv_bfloat16*)nullptr, (float*)nullptr, g,
-                                                                    (__nv_bfloat16*)dX, N);
+                                                                    (__nv_bfloat16*)dX, N, EpiAffine{});
     e = cudaGetLastError();
     if (e != cudaSuccess) { snprintf(g_err, sizeof g_err, "launch: %s", cudaGetErrorString(e)); return 5; }
     g_launches.fetch_add(1);

@@ -452,6 +452,8 @@ extern "C" int sy_ops_bn_bwd_dual(const void* dout, const void* dout2, const voi
 // bwd: one thread per (input pixel, 8-channel group): gathers from the <= 4 windows that cover
 //      it (no atomics, every dx element written exactly once).
 // ===========================================================================
+// kIdx = false: inference variant without the arg-max codes (no index bytes written, no `code` registers)
+template <bool kIdx>
 __global__ void __launch_bounds__(256)
 k_maxpool_fwd(const __nv_bfloat16* __restrict__ x, __nv_bfloat16* __restrict__ y, uint8_t* __restrict__ idx,
               int N, int H, int W, int C, int OH, int OW) {
@@ -474,11 +476,12 @@ k_maxpool_fwd(const __nv_bfloat16* __restrict__ x, __nv_bfloat16* __restrict__ y
         if (ix < 0 || ix >= W) continue;
         float f[8]; unpack8(ldg16(x + (((long)n * H + iy) * W + ix) * C + g * 8), f);
 #pragma unroll
-        for (int i = 0; i < 8; ++i) if (f[i] > best[i]) { best[i] = f[i]; code[i] = ky * 3 + kx; }
+        for (int i = 0; i < 8; ++i) if (f[i] > best[i]) { best[i] = f[i]; if (kIdx) code[i] = ky * 3 + kx; }
       }
     }
     const long o = (((long)n * OH + oy) * OW + ox) * C + g * 8;
     stg16(y + o, pack8(best));
+    if (!kIdx) continue;
     uint2 c2 = make_uint2(code[0] | (code[1] << 8) | (code[2] << 16) | (code[3] << 24), code[4] | (code[5] << 8) | (code[6] << 16) | (code[7] << 24));
     *reinterpret_cast<uint2*>(idx + o) = c2;
   }
@@ -579,12 +582,16 @@ k_maxpool_bwd2(const __nv_bfloat16* __restrict__ dy, const uint8_t* __restrict__
   }
 }
 
+// idx == NULL: inference (no arg-max codes, nothing for a backward pass)
 extern "C" int sy_ops_maxpool3x3s2_fwd(const void* x, void* y, void* idx, int N, int H, int W, int C, void* stream) {
   if (C % 8) return -1;
   const int OH = (H + 2 - 3) / 2 + 1, OW = (W + 2 - 3) / 2 + 1;
   long total = (long)N * OH * OW * (C / 8);
   int blocks = (int)((total + 255) / 256 < 148 * 16 ? (total + 255) / 256 : 148 * 16);
-  k_maxpool_fwd<<<blocks, 256, 0, (cudaStream_t)stream>>>((const __nv_bfloat16*)x, (__nv_bfloat16*)y, (uint8_t*)idx, N, H, W, C, OH, OW);
+  if (idx)
+    k_maxpool_fwd<true><<<blocks, 256, 0, (cudaStream_t)stream>>>((const __nv_bfloat16*)x, (__nv_bfloat16*)y, (uint8_t*)idx, N, H, W, C, OH, OW);
+  else
+    k_maxpool_fwd<false><<<blocks, 256, 0, (cudaStream_t)stream>>>((const __nv_bfloat16*)x, (__nv_bfloat16*)y, nullptr, N, H, W, C, OH, OW);
   COUNT_LAUNCH();
   RET_LAST();
 }
@@ -603,6 +610,79 @@ extern "C" int sy_ops_maxpool3x3s2_bwd(const void* dy, const void* idx, void* dx
   long total = (long)N * H * W * (C / 8);
   int blocks = (int)((total + 255) / 256 < 148 * 16 ? (total + 255) / 256 : 148 * 16);
   k_maxpool_bwd<<<blocks, 256, 0, (cudaStream_t)stream>>>((const __nv_bfloat16*)dy, (const uint8_t*)idx, (__nv_bfloat16*)dx, N, H, W, C, OH, OW);
+  COUNT_LAUNCH();
+  RET_LAST();
+}
+
+// ===========================================================================
+// Inference BatchNorm.  The fold turns every BN layer of a model into a per-channel affine map in ONE launch (one block per
+// layer), reading the parameters and running statistics where they live, so a captured inference graph always applies the
+// current values:  scale = gamma * rsqrt(running_var + eps),  shift = beta - running_mean * scale.
+// bn_infer_apply is the same map as a stand-alone pass for layers whose convolution has no fused epilogue:
+//   out = act(x * scale + shift (+ residual))  on NHWC bf16 [M, C], C % 8 == 0, 16-byte vectors.
+// ===========================================================================
+struct BnFoldEntry {                  // 64 bytes, laid out by ops/fused.py (eight 64-bit words)
+  const __nv_bfloat16* gamma;
+  const __nv_bfloat16* beta;
+  const float* running_mean;
+  const float* running_var;
+  float* scale_out;
+  float* shift_out;
+  long long C;
+  float eps;
+  float pad_;
+};
+
+__global__ void __launch_bounds__(256)
+k_bn_fold(const BnFoldEntry* __restrict__ table) {
+  const BnFoldEntry e = table[blockIdx.x];
+  for (int c = threadIdx.x; c < (int)e.C; c += blockDim.x) {
+    const float sc = __bfloat162float(e.gamma[c]) * rsqrtf(e.running_var[c] + e.eps);
+    e.scale_out[c] = sc;
+    e.shift_out[c] = __bfloat162float(e.beta[c]) - e.running_mean[c] * sc;
+  }
+}
+
+extern "C" int sy_ops_bn_fold(const void* table, int n_layers, void* stream) {
+  if (n_layers <= 0) return 0;
+  k_bn_fold<<<n_layers, 256, 0, (cudaStream_t)stream>>>((const BnFoldEntry*)table);
+  COUNT_LAUNCH();
+  RET_LAST();
+}
+
+__global__ void __launch_bounds__(256)
+k_bn_infer_apply(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ res, __nv_bfloat16* out,
+                 const float* __restrict__ scale, const float* __restrict__ shift, long nvec, int G, int relu) {
+  for (long v = (long)blockIdx.x * blockDim.x + threadIdx.x; v < nvec; v += (long)gridDim.x * blockDim.x) {
+    const int cg = (int)(v % G);
+    const V16 vx = ldg16(x + v * 8);
+    V16 vr{};
+    if (res) vr = ldg16(res + v * 8);
+    const float4 s0 = __ldg(reinterpret_cast<const float4*>(scale) + 2 * cg), s1 = __ldg(reinterpret_cast<const float4*>(scale) + 2 * cg + 1);
+    const float4 t0 = __ldg(reinterpret_cast<const float4*>(shift) + 2 * cg), t1 = __ldg(reinterpret_cast<const float4*>(shift) + 2 * cg + 1);
+    const float s[8] = {s0.x, s0.y, s0.z, s0.w, s1.x, s1.y, s1.z, s1.w};
+    const float t[8] = {t0.x, t0.y, t0.z, t0.w, t1.x, t1.y, t1.z, t1.w};
+    float f[8], r[8];
+    unpack8(vx, f); unpack8(vr, r);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      f[i] = fmaf(f[i], s[i], t[i]) + r[i];
+      if (relu) f[i] = fmaxf(f[i], 0.f);
+    }
+    stg16(out + v * 8, pack8(f));
+  }
+}
+
+// x, res (optional), out: [M, C] bf16, 16-byte aligned; scale / shift: fp32[C], 16-byte aligned.  out may be x (in place).
+extern "C" int sy_ops_bn_infer_apply(const void* x, const void* res, void* out, const float* scale, const float* shift, long M, int C,
+                                     int relu, void* stream) {
+  if (C % 8 || M < 0 || (((uintptr_t)x | (uintptr_t)res | (uintptr_t)out | (uintptr_t)scale | (uintptr_t)shift) & 15)) return -1;
+  const long nvec = M * (C / 8);
+  if (nvec == 0) return 0;
+  long blocks = (nvec + 255) / 256;
+  if (blocks > 148 * 16) blocks = 148 * 16;
+  k_bn_infer_apply<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>((const __nv_bfloat16*)x, (const __nv_bfloat16*)res, (__nv_bfloat16*)out,
+                                                                  scale, shift, nvec, C / 8, relu);
   COUNT_LAUNCH();
   RET_LAST();
 }

@@ -22,6 +22,21 @@ from batch_shipyard_b200.ops.coll import Communicator  # noqa: E402
 from batch_shipyard_b200.parallel.ddp import FusedDataParallelTrainer  # noqa: E402
 
 
+def _held_out(a, rank, nclass):
+    """a.eval_batches x a.batch held-out uint8 NHWC images and labels for this rank (seeded, disjoint from the training seeds)."""
+    n = a.eval_batches * a.batch
+    seed = 555000 + rank
+    if a.model == "lenet":
+        from batch_shipyard_b200.models.lenet import synthetic_digits
+        return synthetic_digits(n, seed=seed)
+    if a.model == "resnet20":
+        from batch_shipyard_b200.models.resnet import synthetic_cifar
+        return synthetic_cifar(n, seed=seed)
+    g = torch.Generator().manual_seed(seed)
+    return (torch.randint(0, 256, (n, a.image, a.image, 3), dtype=torch.uint8, generator=g),
+            torch.randint(0, nclass, (n,), dtype=torch.int64, generator=g))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--steps", type=int, default=30)
@@ -30,6 +45,9 @@ def main():
     ap.add_argument("--model", default="resnet50", choices=["resnet50", "tiny", "lenet", "resnet20"],
                     help="resnet50 (the GPU recipes), tiny (a 4-block ResNet for smoke runs), lenet (the MNIST network of the single-framework CPU recipes, synthetic digits), resnet20 (the CIFAR-10 ResNet of the MXNet / CNTK examples, synthetic CIFAR-shaped images)")
     ap.add_argument("--lr", type=float, default=0.1)
+    ap.add_argument("--eval-batches", type=int, default=0,
+                    help="after training, evaluate on this many held-out seeded batches per rank (FusedDataParallelTrainer.evaluate; "
+                         "the sums of all ranks are reported under \"eval\")")
     a = ap.parse_args()
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
     gpu = os.environ.get("SHIPYARD_GPU", os.environ.get("LOCAL_RANK", "0"))
@@ -94,6 +112,8 @@ def main():
             model.eval()
             xt = (xs.to(tr.dev).float() / 255.0).permute(0, 3, 1, 2).to(tr.static_x.dtype)
             extra["test_accuracy"] = round(float((model(xt).float().argmax(1).cpu() == ys).float().mean()), 4)
+    if a.eval_batches > 0:
+        extra["eval"] = tr.evaluate(*_held_out(a, rank, nclass), batch=a.batch)
     if rank == 0:
         print(json.dumps({"model": a.model, "images_per_sec": round(a.batch * world * a.steps / dt, 1), "world": world, "steps": a.steps,
                           "first_loss": round(losses[0], 4), "last_loss": round(losses[-1], 4), "transport": comm.transport,
